@@ -2,6 +2,7 @@
 """bench.py — kNN queries/sec of the knowledge-base search path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3] [--impl ours|reference] [--no-extras]
+                    [--dump-outputs DIR]
     python bench.py --gpus N --single-process      (no torchrun: ONE process, one rbk_group handle over N GPUs)
 
 A "step" is one pass of the hot path (batched cosine scan + exact top-k) over one batch of
@@ -57,6 +58,15 @@ def load_synth():
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """--dump-outputs: `arrays` (what the timed call returned in its last step) as float64 DIR/<name>.npy.  Slots
+    and counts are integers below 2**53, so float64 holds them exactly; the largest workload writes about 1 MB."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", np.asarray(a).astype(np.float64))
 
 
 def peaks():
@@ -328,7 +338,7 @@ def run_workload(ctx, args, name, wl, main: bool, steps: int):
             with torch.cuda.stream(stream):
                 flush_buf.zero_()
                 ev0.record(stream)
-                flags = searcher.search_device_async(q_dev, k_fetch, args.min_score)[3]
+                out = searcher.search_device_async(q_dev, k_fetch, args.min_score)
                 ev1.record(stream)
             stream.synchronize()
             ms += ev0.elapsed_time(ev1)
@@ -338,10 +348,14 @@ def run_workload(ctx, args, name, wl, main: bool, steps: int):
         # are accumulated on the device by the merge kernel and checked once after the region
         ev0.record(stream)
         for _ in range(steps):
-            flags = searcher.search_device_async(q_dev, k_fetch, args.min_score)[3]
+            out = searcher.search_device_async(q_dev, k_fetch, args.min_score)
         ev1.record(stream)
         barrier()
         ms = ev0.elapsed_time(ev1)
+    flags = out[3]
+    if main and rank == 0 and args.dump_outputs:
+        # copied now: the same-box comparison below runs the search again into the same buffers
+        dump_outputs(args.dump_outputs, {name: t.cpu().numpy() for name, t in zip(("slots", "scores", "counts", "flags"), out)})
     dirty = int(flags[-1].item()) - searcher._dirty_seen     # running count of unproven queries (merge kernel)
     searcher._dirty_seen += dirty
     st1 = ix.stats()
@@ -493,6 +507,8 @@ def run_group(args, name, wl, pk, synth, reduced):
         dev_ms += got[3]
     dt = time.perf_counter() - t0
     t_r1 = time.monotonic()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("slots", "scores", "counts"), got[:3])))
     st1 = grp.stats()
     time.sleep(0.05)
     sampler.window(t_r0, t_r1)
@@ -654,7 +670,15 @@ def main():
                     help="only the main workload (default: also cfg5 at every N and cfg4 at N=8, in `extra_workloads`)")
     ap.add_argument("--min-score", type=float, default=None,
                     help="cosine threshold (the reference's default is 0.5); default: none (-inf), the headline runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed search returned in its last step (slots, "
+                         "scores, counts and, on the device-resident path, flags of the main workload) as "
+                         "float64 DIR/<name>.npy; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference leg keeps no results")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = list(WORKLOADS[args.workload])
     reduced = bool(args.rows)
@@ -695,7 +719,7 @@ def main():
         names = ["cfg5"] + (["cfg4"] if ctx.world == 8 else [])
         for nm in names:
             try:
-                extras[nm] = run_workload(ctx, args, nm, list(WORKLOADS[nm]), main=False, steps=min(args.steps, 20))
+                extras[nm] = run_workload(ctx, args, nm, list(WORKLOADS[nm]), main=False, steps=args.steps)
             except Exception as e:   # an extra must never cost the headline line
                 extras[nm] = {"error": f"{type(e).__name__}: {e}"}
     if ctx.rank == 0:

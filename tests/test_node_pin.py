@@ -1,7 +1,7 @@
 """The pin (SURVEY.md §8c): wherever Node AND a checkout of the reference exist, run the reference's OWN
 cosineSimilarity / findMostSimilar (tests/golden/make_golden_node.mjs) over the inputs of knn_golden.json and require
-the stored outputs bit for bit.  Neither exists in the build image or on the GPU box, so this test skips there and the
-oracle header keeps saying "parity unpinned"; on any developer machine with Node >= 22.6 it is one command."""
+the stored outputs bit for bit.  The checkout is not part of this repository: point RBK_REFERENCE at it.  Without
+Node >= 22.6 and RBK_REFERENCE the test skips and the oracle header keeps saying "parity unpinned"."""
 import json
 import os
 import shutil
@@ -15,9 +15,9 @@ HERE = Path(__file__).resolve().parent
 
 def test_golden_vectors_match_the_reference_itself():
     node = shutil.which("node")
-    ref = Path(os.environ.get("RBK_REFERENCE", "/root/reference"))
-    if node is None or not (ref / "src/knowledge/indexer/embedder.ts").exists():
-        pytest.skip("needs node (>= 22.6, --experimental-strip-types) and a checkout of the reference")
+    ref = os.environ.get("RBK_REFERENCE")
+    if node is None or not ref or not (Path(ref) / "src/knowledge/indexer/embedder.ts").exists():
+        pytest.skip("needs node (>= 22.6, --experimental-strip-types) and RBK_REFERENCE naming a checkout of the reference")
     res = subprocess.run([node, "--experimental-strip-types", "--no-warnings", str(HERE / "golden" / "make_golden_node.mjs"), "--check"],
                          capture_output=True, text=True, timeout=300, env=dict(os.environ, RBK_REFERENCE=str(ref)))
     assert res.returncode == 0, res.stdout + res.stderr
