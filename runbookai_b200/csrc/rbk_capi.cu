@@ -333,8 +333,7 @@ rbk_status run_scan(rbk_index* ix, const void* d_q, int src_type, int B, int k_f
   ix->stats.last_kprime = kprime;
   // (also zeroes the scan scratch of the first sub-batch; normA is left to the finalize kernel)
   const int Bs0 = std::min(kMaxSubBatch, B);
-  CK(launch_prep_queries(d_q, src_type, B, ix->dim, ix->dpad, min_score,
-                         ix->keep_f64 ? reinterpret_cast<const float*>(ix->d_counter + 1) : nullptr,
+  CK(launch_prep_queries(d_q, src_type, B, ix->dim, ix->dpad, min_score, reinterpret_cast<const float*>(ix->d_counter + 1),
                          query_buffers(ix, 0), ix->stream, /*with_norm2=*/d_counts == nullptr, ix->hist.p, Bs0,
                          ix->sm_count + 8));
   ix->stats.kernel_launches++;

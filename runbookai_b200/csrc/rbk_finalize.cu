@@ -77,7 +77,27 @@ __global__ void __launch_bounds__(128) prep_queries_kernel(const SrcT* __restric
       for (int i = tid; i < n_progress; i += blockDim.x) tail[2 * Bs + i] = 0u;
   }
   const SrcT* s = src + static_cast<size_t>(q) * d;
-  double sb = 0.0, sd = 0.0, sq = 0.0;  // ||bf16(q)||^2, ||q - bf16(q)||^2, ||q||^2 (any order: bounds only)
+  // The scan's copy is bf16(q * 2^e), e chosen so that the largest |element| lands in [1, 2) (DESIGN.md §6: every
+  // tensor-core product and partial sum is then a normal fp32 number for rows inside the norm window, whatever the
+  // query's own scale - cosine does not depend on it).  Scaling by 2^e is exact in fp64.  q_f64, normA and the
+  // validity test stay on the unscaled query: they define the reference's result.
+  __shared__ double red_m[4];
+  double amax = 0.0;
+  for (int i0 = tid; i0 < d; i0 += 8 * blockDim.x) {
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      const int i = i0 + u * blockDim.x;
+      if (i < d) amax = fmax(amax, fabs(static_cast<double>(__ldg(s + i))));
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) amax = fmax(amax, __shfl_xor_sync(kFull, amax, o));
+  if ((tid & 31) == 0) red_m[tid >> 5] = amax;
+  __syncthreads();
+  amax = fmax(fmax(red_m[0], red_m[1]), fmax(red_m[2], red_m[3]));
+  const int e = (amax > 0.0 && amax < INFINITY) ? -ilogb(amax) : 0;
+  // ||bf16(qs)||^2, ||qs - bf16(qs)||^2, ||qs||^2 of the scaled copy qs (any order: bounds only); ||q||^2 unscaled
+  double sb = 0.0, sd = 0.0, ss = 0.0, sq = 0.0;
   // 8 elements per thread and pass, ALL loads first: the stores below may alias the source as far as the compiler
   // knows, so a load -> store loop exposed one global round trip per element (the kernel took 7.8 us for this)
   for (int i0 = tid; i0 < dpad; i0 += 8 * blockDim.x) {
@@ -95,26 +115,30 @@ __global__ void __launch_bounds__(128) prep_queries_kernel(const SrcT* __restric
       if (i < d) {
         const double x = xs[u];
         qb.q_f64[static_cast<size_t>(q) * d + i] = x;
-        const __nv_bfloat16 h = __float2bfloat16_rn(__double2float_rn(x));
+        const double xs2 = scalbn(x, e);
+        const __nv_bfloat16 h = __float2bfloat16_rn(__double2float_rn(xs2));
         b = __bfloat16_as_ushort(h);
         const double xb = static_cast<double>(__bfloat162float(h));
         sb += xb * xb;
-        sd += (x - xb) * (x - xb);
+        sd += (xs2 - xb) * (xs2 - xb);
+        ss += xs2 * xs2;
         sq += x * x;
       }
       qb.q_bf16[static_cast<size_t>(q) * dpad + i] = b;
     }
   }
-  __shared__ double red_b[4], red_d[4];
+  __shared__ double red_b[4], red_d[4], red_s[4];
   __shared__ double s_na;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     sb += __shfl_xor_sync(kFull, sb, o);
     sd += __shfl_xor_sync(kFull, sd, o);
+    ss += __shfl_xor_sync(kFull, ss, o);
   }
   if ((tid & 31) == 0) {
     red_b[tid >> 5] = sb;
     red_d[tid >> 5] = sd;
+    red_s[tid >> 5] = ss;
   }
   // the reference's normA: index order, multiply then add.  The chain is sequential by contract, so its
   // operands are staged in smem first (a dependent global load per element cost ~23 ns each).
@@ -145,16 +169,17 @@ __global__ void __launch_bounds__(128) prep_queries_kernel(const SrcT* __restric
     const double na = s_na;
     const double nb2 = red_b[0] + red_b[1] + red_b[2] + red_b[3];
     const double nd2 = red_d[0] + red_d[1] + red_d[2] + red_d[3];
+    const double ns2 = red_s[0] + red_s[1] + red_s[2] + red_s[3];
     const bool ok = nb2 > 0.0 && nb2 < INFINITY && na > 0.0 && na < INFINITY;
     const double inv = ok ? 1.0 / sqrt(nb2) : 0.0;
-    // angle(q, bf16(q)) <= asin(||q - bf16(q)|| / ||q||); cosine is 1-Lipschitz in the angle
+    // angle(qs, bf16(qs)) <= asin(||qs - bf16(qs)|| / ||qs||); cosine is 1-Lipschitz in the angle
     double ang = 0.0;
     if (ok && nd2 > 0.0) {
-      const double ratio = sqrt(nd2 / na) * (1.0 + 1e-9) * (kNorm2 ? 1.0 : 1.0 + 1e-12 * d);   // any-order sum: widen
-
+      const double ratio = sqrt(nd2 / ns2) * (1.0 + 1e-9) * (1.0 + 1e-12 * d);   // any-order sums: widen
       ang = ratio < 1.0 ? asin(ratio) * (1.0 + 1e-9) : 3.2;
     }
-    // + corpus-side quantisation angle when the exact source is an f64 sidecar (0 for bf16-exact corpora)
+    // + corpus-side term (rbk_ingest.cu): the quantisation angle of an f64 sidecar's rows, and 3.2 (no bound) once
+    // a row's norm has left the scan's window; 0 for bf16-exact corpora inside the window
     const double eps = acc_eps + ang + (eps_c != nullptr ? static_cast<double>(*eps_c) * (1.0 + 1e-6) : 0.0);
     if (kNorm2) qb.q_norm2[q] = na;   // (else: written by the finalize kernel, bit-exact)
     qb.q_eps[q] = eps;
@@ -499,7 +524,11 @@ __global__ void __launch_bounds__(kFinThreads) finalize_kernel(FinalizeParams p)
     p.out_counts[ql] = count;
     // ---- proof of exactness (DESIGN.md §6) ----
     bool ok;
-    if (tau_raw == -INFINITY) {
+    if (!(p.q.q_eps[ql] < 2.0)) {
+      // cosines lie in [-1, 1]: a bound this wide (a row outside the scan's norm window, DESIGN.md §6) says nothing
+      // about the rows the scan dropped - NaN accumulators included - so nothing is proven
+      ok = false;
+    } else if (tau_raw == -INFINITY) {
       ok = true;  // nothing was ever dropped except by thr_init (provably below min_score)
     } else {
       const double bound = static_cast<double>(tau_raw) * static_cast<double>(p.q.q_inv_norm[ql]) + p.q.q_eps[ql];

@@ -128,6 +128,7 @@ __device__ __forceinline__ double bf16_bits_to_f64(uint32_t h) {
 constexpr int kNormRows = 128;          // rows (= threads) per block
 constexpr int kNormChunk = 128;         // bf16 elements per staged chunk (256 B per row)
 constexpr int kNormPitch16 = kNormChunk / 8 + 1;   // 17 x 16 B per row in smem: odd -> conflict-free walks
+constexpr double kNormLo = 0x1p-60, kNormHi = 0x1p100;   // the scan's row-norm window
 
 __global__ void __launch_bounds__(kNormRows) row_norms_kernel(const uint16_t* __restrict__ rows_base,
                                                               const double* __restrict__ rows_f64_base,
@@ -207,6 +208,10 @@ __global__ void __launch_bounds__(kNormRows) row_norms_kernel(const uint16_t* __
   const bool ok = acc > 0.0 && acc < INFINITY;
   inv_norm_base[my_row] = ok ? static_cast<float>(1.0 / sqrt(acc)) : __uint_as_float(0x7FC00000u);
   if (rows_f64_base == nullptr) norm2_base[my_row] = acc;
+  // The scan's error bound holds for ||row|| in [kNormLo, kNormHi] (DESIGN.md §6): outside it the fp32 accumulator
+  // may overflow or lose products to underflow.  Such a row voids the bound for the whole index (3.2 > any cosine
+  // distance), so every proof fails and the exhaustive fp64 kernel answers.
+  if (ok && !(acc >= kNormLo * kNormLo && acc <= kNormHi * kNormHi)) atomicMax(eps_c_max, __float_as_int(3.2f));
 }
 
 // Exact-source sidecar indexes (RBK_INDEX_KEEP_F64): norm2 comes from the f64 row (the reference's normB for

@@ -101,7 +101,8 @@ cudaError_t launch_convert_rows(const void* src, int src_type, int64_t n_rows, i
                                 int* n_dead = nullptr);
 // Norms of rows [first_row, first_row + n_items) of the index (or, with slot_map, of rows slot_map[i]; tombstoned
 // ones skipped).  All array arguments are the index's BASE pointers.  rows_f64_base (nullable): when given,
-// norm2 comes from it and the bf16-vs-f64 angle bound is max-ed into *eps_c_max (float bits in an int).
+// norm2 comes from it and the bf16-vs-f64 angle bound is max-ed into *eps_c_max (float bits in an int).  Any index:
+// a row whose norm is outside the scan's window (DESIGN.md §6) max-es 3.2 into *eps_c_max.
 cudaError_t launch_row_norms(const uint16_t* rows_base, const double* rows_f64_base, int64_t first_row,
                              int64_t n_items, int d, int dpad, float* inv_norm_base, double* norm2_base,
                              int* eps_c_max, cudaStream_t stream, const int64_t* slot_map = nullptr,
@@ -114,12 +115,13 @@ struct QueryBuffers {
   uint16_t* q_bf16;    // [B][dpad]
   double* q_f64;       // [B][d]
   double* q_norm2;     // [B] exact sequential sum of squares of the f64 query (reference's normA)
-  float* q_inv_norm;   // [B] 1/||bf16(q)||  (approximate-score scaling)
+  float* q_inv_norm;   // [B] 1/||bf16(q * 2^e)||, e per query (approximate-score scaling of the scan's copy)
   double* q_eps;       // [B] bound on |approx - exact| cosine for this query
   float* thr_init;     // [B]
 };
 // src_type: 0 = f64, 1 = f32 (device pointers, row pitch d)
-// eps_c (nullable): device float, bound on the corpus-side quantisation angle (f64 sidecar indexes).
+// eps_c (nullable): device float, corpus-side term of the error bound (rbk_ingest.cu: the quantisation angle of f64
+// sidecar rows; 3.2 once a row's norm has left the scan's window).
 // with_norm2: also run the sequential normA chain (only the exact-scores path, which has no finalize kernel; a
 // search leaves it to finalize).  scratch (nullable): hist | maxbin | gthr | progress of the first sub-batch (Bs
 // queries, n_progress pacing slots), zeroed by the kernel.
